@@ -49,7 +49,53 @@ def parse():
     ap.add_argument("--nulls", type=int, default=0, help="mixed workload: null permille of every column (50 = the 5 %% variant)")
     ap.add_argument("--no-verify", action="store_true", help="skip the answer check after the timed loop")
     ap.add_argument("--verify-series", type=int, default=4, help="series sampled for the bitwise check against the oracle")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the arrays the last step returned as DIR/<name>.npy "
+                                                          "(float64 / float32, at most 64 MB in all) to compare two builds output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path returned: it needs --impl ours")
+    return a
+
+
+DUMP_LIMIT = 60_000_000  # bytes of array data: the files stay under 64 MB with their .npy headers
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Write {name: array} as out_dir/<name>.npy.  Integers and float64 go out as float64 (an integer that float64 cannot hold
+    exactly is an error: times are passed as offsets from T0), bytes and flags as float32.  While the whole exceeds `limit`, the
+    largest array is replaced by its elements at sorted positions drawn with a fixed seed; the positions go to <name>_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a).ravel()
+        f = a.astype(np.float32 if a.dtype.itemsize <= 2 else np.float64)
+        if a.dtype.kind in "iub" and not np.array_equal(f.astype(a.dtype), a):
+            raise ValueError(f"--dump-outputs: {name} holds integers that {f.dtype} cannot represent exactly")
+        out[name] = f
+    while sum(v.nbytes for v in out.values()) > limit:
+        name = max((k for k in arrays if k + "_index" not in out), key=lambda k: out[k].nbytes)
+        v = out[name]
+        room = limit - (sum(x.nbytes for x in out.values()) - v.nbytes)
+        m = max(1, room // (v.itemsize + 8))
+        idx = np.sort(np.random.default_rng(0).choice(v.size, size=min(m, v.size - 1), replace=False))
+        out[name], out[name + "_index"] = v[idx], idx.astype(np.float64)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
+def dense_arrays(d, calls):
+    """The dense interval record a query returns (AggQuery.dense_host()), one array per field; times relative to T0."""
+    import numpy as np
+    arrays = {"grid": np.array([d["n_groups"], d["n_buckets"], d["start"] - T0, d["interval"]], np.int64)}
+    for (func, col), c in zip(calls, d["cols"]):
+        arrays[f"{func}_f{col}_values"] = c["values"]
+        arrays[f"{func}_f{col}_valid"] = c["valid"]
+        if c["times"] is not None:
+            arrays[f"{func}_f{col}_times"] = c["times"] - T0
+    return arrays
 
 
 class ClockSampler:
@@ -406,6 +452,8 @@ def run_ours(a):
         dist.barrier()
     wall_s = time.perf_counter() - w0
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, dense_arrays(q.dense_host(), calls))
     t = torch.tensor([dev_ms, wall_s * 1e3], dtype=torch.float64, device=dev)
     rows_t = torch.tensor([float(st["rows_decoded"])], dtype=torch.float64, device=dev)
     if world > 1:
@@ -605,6 +653,8 @@ def run_mixed(a):
         q.run(); st = q.stats()
         dev_ms += st["kernel_ms"]; main_ms += st["main_kernel_ms"]; launches += st["kernel_launches"]
     clocks = sampler.stop()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, dense_arrays(q.dense_host(), calls))
     # answer check on a slice: the first K series of the population, same seed, through the oracle
     verify = None
     if not a.no_verify:
@@ -665,6 +715,14 @@ def run_downsample(a):
         out = downsample(sh, 0, ivl, T0, tmax)
     torch.cuda.synchronize(); wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if a.dump_outputs:
+        # the new shard as the pass hands it back: page bytes and their directory (window times relative to T0)
+        arrays = {"pages": out["data"][:out["data_len"]].cpu().numpy(), "sids": out["sids"], "series_seg_begin": out["series_seg_begin"],
+                  "seg_tmin": out["seg_tmin"] - T0, "seg_tmax": out["seg_tmax"] - T0,
+                  "time_page_off": out["time_page_off"], "time_page_len": out["time_page_len"]}
+        for name, _typ, po, pl in out["columns"]:
+            arrays[f"{name}_page_off"], arrays[f"{name}_page_len"] = po, pl
+        dump_outputs(a.dump_outputs, arrays)
     verify = None
     if not a.no_verify:
         host = out["data"].cpu().numpy()[:out["data_len"]].copy()
